@@ -113,6 +113,25 @@ int jqc_build_partial(jqc_engine* eng, const double* dm_dev, int n_dm, int hermi
                       size_t* partial_len, void* stream);
 int jqc_finalize(jqc_engine* eng, double* vj_dev, double* vk_dev, void* stream);
 
+/* Nuclear gradient of the J/K energy for one symmetric density D (molecule AO basis, FP64):
+ *     E_jk(R) = (j_factor / 2) tr(D J[D]) - (k_factor / 4) tr(D K[D])
+ * with J, K exactly what jqc_get_jk(hermi = 1, omega) returns; D is held fixed and the basis
+ * functions move with their atoms.  grad_dev (natm x 3, device, Hartree/Bohr) is written with
+ * g[A, x] = dE_jk / dR_{A,x}.  RHF: j_factor = k_factor = 1; hybrid: k_factor = hyb; the long-range
+ * part of a range-separated hybrid is a second call with omega > 0, j_factor = 0,
+ * k_factor = alpha - hyb.  shell_atom (HOST, nbas): atom of each kernel-side shell, -1 for pads.
+ * Quartets are screened with q_ij + q_kl + max(d_ij + d_kl [j_factor != 0], d_ik + d_jl,
+ * d_il + d_jk [k_factor != 0]) > log(cutoff) in float32 logs.  With a shard set
+ * (jqc_engine_set_shard) the call writes this rank's partial gradient; the caller sums the ranks.
+ * quartets (may be NULL): if given, the call synchronises and stores the number of quartets
+ * evaluated.  JQC_EINVAL for omega < 0, j_factor == k_factor == 0, cutoff <= 0, natm < 1 or a
+ * shell_atom entry outside [-1, natm).  The state of the last J/K build is left alone, so
+ * jqc_build_partial -> jqc_jk_energy_grad -> jqc_finalize still finalises that build; scratch is
+ * shared with the J/K builds, so calls on one engine are issued in stream order. */
+int jqc_jk_energy_grad(jqc_engine* eng, const double* dm_dev, double j_factor, double k_factor,
+                       double omega, double cutoff, const int* shell_atom, int natm, double* grad_dev,
+                       long long* quartets, void* stream);
+
 /* Accounting of the last build (synchronises the engine's device).  counts: 625 entries,
  * quartets evaluated per class key ((li*5+lj)*5+lk)*5+ll; prim_weighted: the same weighted by
  * npi*npj*npk*npl (for the algorithmic FLOP model of SURVEY 8d); launches: kernels enqueued. */

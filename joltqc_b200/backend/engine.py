@@ -161,6 +161,33 @@ class JKEngine:
         dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=group)
         return buf
 
+    def jk_energy_grad(self, dm, shell_atom, natm, j_factor=1.0, k_factor=1.0, omega=None, cutoff=1e-13, group=None,
+                       count=False):
+        """Nuclear gradient of E_jk = (j_factor/2) tr(D J[D]) - (k_factor/4) tr(D K[D]) for one symmetric
+        density ``dm`` (mol_nao x mol_nao, molecule AO basis) as a (natm, 3) float64 device tensor
+        (jqc_jk_energy_grad).  ``shell_atom``: BasisLayout.shell_atom.  With sharding enabled the partial
+        gradients of all ranks are summed with one all_reduce, as in get_jk.  ``count=True`` also stores
+        the number of quartets this rank evaluated in ``self.last_grad_quartets`` (synchronises)."""
+        d = self._dev(dm)
+        if d.ndim != 2 or d.shape[0] != self.mol_nao or d.shape[1] != self.mol_nao:
+            raise ValueError(f"dm has shape {tuple(d.shape)}, expected ({self.mol_nao}, {self.mol_nao})")
+        sa = np.ascontiguousarray(shell_atom, dtype=np.int32)
+        if sa.shape != (self.nbas,):
+            raise ValueError(f"shell_atom has shape {sa.shape}, expected ({self.nbas},)")
+        out = torch.empty((int(natm), 3), dtype=torch.float64, device=self.device)
+        nq = ctypes.c_longlong(0)
+        with torch.cuda.device(self.device):
+            _lib.check(self.L.jqc_jk_energy_grad(self.h, d.data_ptr(), float(j_factor), float(k_factor),
+                                                 0.0 if omega is None else float(omega), float(cutoff),
+                                                 _ptr(sa, ctypes.c_int), int(natm), out.data_ptr(),
+                                                 ctypes.byref(nq) if count else None, self._stream()))
+            if count:
+                self.last_grad_quartets = int(nq.value)
+            if getattr(self, "_world", 1) > 1:
+                import torch.distributed as dist
+                dist.all_reduce(out, op=dist.ReduceOp.SUM, group=group)
+        return out
+
     def get_jk_host(self, dm, hermi=0, with_j=True, with_k=True, omega=None, cutoff_fp64=1e-13, cutoff_fp32=1e-13,
                     out=None):
         """Host-buffer entry point (numpy in, numpy out): H2D + build + D2H inside the C call

@@ -1,8 +1,8 @@
 """In-tree build of the CUDA library (libjoltqc_b200.so) for sm_100a.
 
-nvcc is driven directly (no cmake): one object per bra class from csrc/jk_inst.cu plus the
-engine, linked into joltqc_b200/libjoltqc_b200.so.  Objects are cached under
-joltqc_b200/_build/ and rebuilt when any csrc file is newer.
+nvcc is driven directly (no cmake): one object per bra class from csrc/jk_inst.cu (J/K) and from
+csrc/jk_grad_inst.cu (J/K energy gradient) plus the engine, linked into joltqc_b200/libjoltqc_b200.so.
+Objects are cached under joltqc_b200/_build/ and rebuilt when any csrc file is newer.
 """
 import os
 import subprocess
@@ -44,11 +44,12 @@ def build(force=False, verbose=False, jobs=None, extra_flags=None, out=None, obj
     stamp = _newest_src()
     todo = []
     objs = []
-    for i, j in BRA:
-        o = os.path.join(OBJ, f"jk_inst_{i}{j}.o")
-        objs.append(o)
-        if force or not os.path.exists(o) or os.path.getmtime(o) < stamp:
-            todo.append([NVCC] + FLAGS + [f"-DJQC_LI={i}", f"-DJQC_LJ={j}", "-c", os.path.join(CSRC, "jk_inst.cu"), "-o", o])
+    for unit in ("jk_inst", "jk_grad_inst"):
+        for i, j in BRA:
+            o = os.path.join(OBJ, f"{unit}_{i}{j}.o")
+            objs.append(o)
+            if force or not os.path.exists(o) or os.path.getmtime(o) < stamp:
+                todo.append([NVCC] + FLAGS + [f"-DJQC_LI={i}", f"-DJQC_LJ={j}", "-c", os.path.join(CSRC, unit + ".cu"), "-o", o])
     o = os.path.join(OBJ, "engine.o")
     objs.append(o)
     if force or not os.path.exists(o) or os.path.getmtime(o) < stamp:

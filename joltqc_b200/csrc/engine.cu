@@ -20,6 +20,7 @@
 #include "../../include/joltqc_b200.h"
 #include "engine_kernels.cuh"
 #include "jk_brick.cuh"
+#include "jk_grad.cuh"
 #include "jk_launch.h"
 
 using namespace jqc;
@@ -108,6 +109,12 @@ struct jqc_engine {
     DevBuf<ushort4> d_queue;
     DevBuf<unsigned> d_counters;
     DevBuf<unsigned long long> d_qcounts;
+    // energy gradient (jqc_jk_energy_grad): own task counters, so that the accounting of the last J/K
+    // build stays readable, plus the per-shell accumulator and the shell -> atom map
+    DevBuf<unsigned> d_gcounters;
+    DevBuf<unsigned long long> d_gqcounts;
+    DevBuf<double> d_gshell;
+    DevBuf<int> d_gatom;
     int rank = 0, world = 1;
     // task format for blocks of <= 81 integrals: 0 flat quartets (default), 1 4x4 tile records.
     // Both were measured in round 1 (profiles/README.md); JQC_SMALL_TILES=1 selects the tile kernel.
@@ -701,7 +708,7 @@ extern "C" int jqc_build_partial(jqc_engine* e, const double* dm_dev, int n_dm, 
                 CU(cudaEventRecord(e0, st));
             }
             dim3 sgrid((s.kl_count + 31) / 32, (s.ij_count * 16 + 7) / 8);
-            screen_tasks_kernel<<<sgrid, dim3(32, 8), 0, st>>>(s);
+            screen_tasks_kernel<false><<<sgrid, dim3(32, 8), 0, st>>>(s);
             CU(cudaGetLastError());
             JKArgs a;
             a.nao = nao;
@@ -730,6 +737,143 @@ extern "C" int jqc_build_partial(jqc_engine* e, const double* dm_dev, int n_dm, 
     e->built = true;
     if (partial_dev) *partial_dev = e->d_vjk.p;
     if (partial_len) *partial_len = 2 * neff * nao2;
+    return JQC_OK;
+}
+
+// ---------------------------------------------------------------------------------------
+// Nuclear gradient of E_jk = (j_factor/2) tr(D J[D]) - (k_factor/4) tr(D K[D]) (include/joltqc_b200.h).
+// Same front end as a J/K build (transform in, pooling, active tile lists, chunked group-quartet loop
+// with the device queue), on the quartet-list path only.  The density scratch, the pooled density and the
+// queue are shared with the J/K builds (stream-ordered); the [J || K] buffer, the chunk records and the
+// task counters that jqc_finalize and jqc_last_stats read are not touched.
+extern "C" int jqc_jk_energy_grad(jqc_engine* e, const double* dm_dev, double j_factor, double k_factor, double omega,
+                                  double cutoff, const int* shell_atom, int natm, double* grad_dev, long long* quartets,
+                                  void* stream)
+{
+    if (!e || !dm_dev || !shell_atom || !grad_dev) return fail(JQC_EINVAL, "null argument");
+    if (omega < 0) return fail(JQC_EINVAL, "short ranged J/K not supported");
+    if (j_factor == 0.0 && k_factor == 0.0) return fail(JQC_EINVAL, "j_factor or k_factor must be non-zero");
+    if (!(cutoff > 0)) return fail(JQC_EINVAL, "cutoff must be positive");
+    if (natm < 1) return fail(JQC_EINVAL, "natm must be >= 1");
+    for (int s = 0; s < e->nbas; s++)
+        if (shell_atom[s] < -1 || shell_atom[s] >= natm) return fail(JQC_EINVAL, "shell_atom entry outside [-1, natm)");
+    CU(cudaSetDevice(e->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    QData* qd = nullptr;
+    int rc = get_qdata(e, omega, &qd);
+    if (rc) return rc;
+
+    const int nao = e->nao, nbas = e->nbas, npairs = e->npairs();
+    const size_t nao2 = (size_t)nao * nao;
+    CU(e->d_dm.ensure(std::max<size_t>(nao2, 1)));
+    CU(e->d_cond.ensure((size_t)nbas * nbas));
+    CU(e->d_logd.ensure((size_t)nbas * nbas));
+    CU(e->d_gcounters.ensure(MAX_CHUNKS));
+    CU(e->d_gqcounts.ensure(MAX_CHUNKS));
+    CU(e->d_gshell.ensure((size_t)nbas * 3));
+    CU(e->d_gatom.ensure(nbas));
+    CU(cudaMemcpyAsync(e->d_gatom.p, shell_atom, nbas * sizeof(int), cudaMemcpyHostToDevice, st));
+
+    // 1. AO transform in, 2. pooling (hermi = 1), log, global max, 3. active tile counts (quadratic in D)
+    rc = launch_from_mol(e, dm_dev, 1, e->d_dm.p, false, st);
+    if (rc) return rc;
+    dm_pool_kernel<<<nbas, 256, nbas * sizeof(float), st>>>(e->d_dm.p, 1, nao, nbas, e->d_ao_loc.p, e->d_ao2shell.p,
+                                                          e->d_cond.p);
+    CU(cudaGetLastError());
+    {
+        const int neg_inf_ordered = (int)0xFF800000 ^ 0x7FFFFFFF;   // float_to_ordered(-inf)
+        CU(cudaMemcpyAsync(e->d_logmax.p, &neg_inf_ordered, sizeof(int), cudaMemcpyHostToDevice, st));
+        dim3 grid(nbas, (nbas + 127) / 128);
+        dm_log_kernel<<<grid, 128, 0, st>>>(e->d_cond.p, nbas, 1, e->d_logd.p, e->d_logmax.p);
+        CU(cudaGetLastError());
+    }
+    active_tiles_grad_kernel<<<(npairs + 127) / 128, 128, 0, st>>>(qd->tiles_q.p, qd->list_off.p, npairs, e->d_logmax.p,
+                                                                  e->d_nact.p);
+    CU(cudaGetLastError());
+    CU(cudaMemsetAsync(e->d_gshell.p, 0, (size_t)nbas * 3 * sizeof(double), st));
+    CU(cudaMemsetAsync(e->d_gcounters.p, 0, MAX_CHUNKS * sizeof(unsigned), st));
+    CU(cudaMemsetAsync(e->d_gqcounts.p, 0, MAX_CHUNKS * sizeof(unsigned long long), st));
+    std::vector<int> nact(npairs);
+    CU(cudaMemcpyAsync(nact.data(), e->d_nact.p, npairs * sizeof(int), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+
+    // 4. group-quartet loop of the quartet-list path (jqc_build_partial), heavy classes first
+    const float log_cut = (float)std::log(cutoff);
+    int nchunks = 0;
+    bool queue_ready = false;
+    for (int gi = e->ngroups - 1; gi >= 0; gi--)
+    for (int gj = gi; gj >= 0; gj--)
+    for (int gk = gi; gk >= 0; gk--)
+    for (int gl = gk; gl >= 0; gl--) {
+        const int pij = jqc_engine::pair_id(gi, gj), pkl = jqc_engine::pair_id(gk, gl);
+        const int n_ij_all = nact[pij];
+        const int n_kl = nact[pkl];
+        if (n_ij_all == 0 || n_kl == 0) continue;
+        const int li = e->gl[gi], lj = e->gl[gj], lk = e->gl[gk], ll = e->gl[gl];
+        const int n_ij = (n_ij_all + e->world - 1) / e->world;
+        if (n_ij <= 0) continue;
+        const int kl_chunk = std::min({n_kl, e->kl_chunk_max, (int)(e->queue_cap / 256)});
+        const int ij_chunk = std::max(1, (int)std::min<size_t>({(size_t)n_ij, e->queue_cap / 256 / kl_chunk, (size_t)32767}));
+        if (!queue_ready) {
+            const size_t mx = (size_t)*std::max_element(nact.begin(), nact.end());
+            CU(e->d_queue.ensure(std::max<size_t>(256, std::min(e->queue_cap, 256 * mx * std::min<size_t>(mx, e->kl_chunk_max)))));
+            queue_ready = true;
+        }
+        for (int ij0 = 0; ij0 < n_ij; ij0 += ij_chunk)
+        for (int kl0 = 0; kl0 < n_kl; kl0 += kl_chunk) {
+            if (nchunks >= MAX_CHUNKS) return fail(JQC_ENOMEM, "too many task chunks");
+            const int cid = nchunks++;
+            ScreenArgs s;
+            s.nbas = nbas;
+            s.q = qd->q.p;
+            s.logd = e->d_logd.p;
+            s.log_max_ordered = e->d_logmax.p;
+            s.tiles_ij = qd->tiles.p + qd->h_list_off[pij];
+            s.tiles_kl = qd->tiles.p + qd->h_list_off[pkl];
+            s.tileq_kl = qd->tiles_q.p + qd->h_list_off[pkl];
+            s.nact_ij = e->d_nact.p + pij;
+            s.nact_kl = e->d_nact.p + pkl;
+            s.ij_begin = ij0;
+            s.ij_count = std::min(ij_chunk, n_ij - ij0);
+            s.kl_begin = kl0;
+            s.kl_count = std::min(kl_chunk, n_kl - kl0);
+            s.rank = e->rank;
+            s.world = e->world;
+            s.cutoff = log_cut;
+            s.do_j = j_factor != 0.0;
+            s.do_k = k_factor != 0.0;
+            s.queue = e->d_queue.p;
+            s.counter = e->d_gcounters.p + cid;
+            s.qcount = e->d_gqcounts.p + cid;
+            s.tile_mode = 0;
+            dim3 sgrid((s.kl_count + 31) / 32, (s.ij_count * 16 + 7) / 8);
+            screen_tasks_kernel<true><<<sgrid, dim3(32, 8), 0, st>>>(s);
+            CU(cudaGetLastError());
+            GradArgs a;
+            a.nao = nao;
+            a.npi = e->gnp[gi]; a.npj = e->gnp[gj]; a.npk = e->gnp[gk]; a.npl = e->gnp[gl];
+            a.basis = e->d_basis.p;
+            a.dm = e->d_dm.p;
+            a.j_factor4 = 4.0 * j_factor;
+            a.k_factor = k_factor;
+            a.omega = omega;
+            a.quartets = e->d_queue.p;
+            a.ntasks = e->d_gcounters.p + cid;
+            a.gshell = e->d_gshell.p;
+            CU(jk_grad_launch(li, lj, lk, ll, a, e->nsm, st));
+        }
+    }
+    // 5. shells -> atoms
+    grad_shell_to_atom_kernel<<<(3 * natm + 127) / 128, 128, 0, st>>>(e->d_gshell.p, e->d_gatom.p, nbas, natm, grad_dev);
+    CU(cudaGetLastError());
+    if (quartets) {
+        std::vector<unsigned long long> h(std::max(nchunks, 1), 0ull);
+        if (nchunks) CU(cudaMemcpyAsync(h.data(), e->d_gqcounts.p, nchunks * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        long long n = 0;
+        for (int c = 0; c < nchunks; c++) n += (long long)h[c];
+        *quartets = n;
+    }
     return JQC_OK;
 }
 

@@ -87,6 +87,23 @@ __global__ void active_tiles_kernel(const float* __restrict__ list_q, const int*
     n_active[p] = lo - base;
 }
 
+// The same count for the energy-gradient screen, whose density factor is quadratic: the pair cutoff
+// is log(1e-13) - 2 log_max_dm.
+__global__ void active_tiles_grad_kernel(const float* __restrict__ list_q, const int* __restrict__ list_off, int npairs,
+                                         const int* __restrict__ log_max_ordered, int* __restrict__ n_active)
+{
+    const int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= npairs) return;
+    const double cutoff = log(1e-13) - 2.0 * (double)ordered_to_float(*log_max_ordered);
+    int lo = list_off[p], hi = list_off[p + 1];
+    const int base = lo;
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if ((double)list_q[mid] > cutoff) lo = mid + 1; else hi = mid;
+    }
+    n_active[p] = lo - base;
+}
+
 // ------------------------------------------------------------------ task generation
 struct ScreenArgs {
     int nbas;
@@ -113,6 +130,10 @@ struct ScreenArgs {
 // reference's canonical order and float32 log-domain criterion
 // (jqc/backend/jk/screen_jk_tasks.cu:196-261), compacted per warp with one atomic.
 // A warp holds 32 kl tiles for a single (i,j), so its output run shares i and j.
+// GRAD selects the screen of the J/K energy gradient, whose weights are products of two density
+// blocks: q_ij + q_kl + max(d_ij + d_kl [J], d_ik + d_jl, d_il + d_jk [K]) > cutoff, with the tile
+// prefilter on 2 log max|D| (flat quartet records only).
+template <bool GRAD>
 __global__ void __launch_bounds__(256) screen_tasks_kernel(const ScreenArgs s)
 {
     const int nbas = s.nbas, nt = nbas / TILE;
@@ -136,7 +157,7 @@ __global__ void __launch_bounds__(256) screen_tasks_kernel(const ScreenArgs s)
         tl = tkl - tk * nt;
         q_ij = s.q[(size_t)ish * nbas + jsh];
         active = ish >= jsh && tk * TILE <= ish &&
-                 (q_ij + s.tileq_kl[s.kl_begin + kl_slot] + log_max > s.cutoff);
+                 (q_ij + s.tileq_kl[s.kl_begin + kl_slot] + (GRAD ? 2.f * log_max : log_max) > s.cutoff);
     }
     unsigned mask = 0;
     if (active) {
@@ -160,19 +181,30 @@ __global__ void __launch_bounds__(256) screen_tasks_kernel(const ScreenArgs s)
                 const int lsh = lsh0 + l;
                 if (ksh > ish || lsh > ksh || bas_ij < (long long)ksh * nbas + lsh) continue;
                 const float q_ijkl = q_ij + qkl[l];
-                float d_large = -36.8f;
-                if (s.do_k) {
-                    d_large = fmaxf(d_large, dik[k]);
-                    d_large = fmaxf(d_large, djk[k]);
-                    d_large = fmaxf(d_large, dil[l]);
-                    d_large = fmaxf(d_large, djl[l]);
+                if constexpr (GRAD) {
+                    float d_large = -73.6f;
+                    if (s.do_j) d_large = fmaxf(d_large, d_ij + dkl[l]);
+                    if (s.do_k) {
+                        d_large = fmaxf(d_large, dik[k] + djl[l]);
+                        d_large = fmaxf(d_large, dil[l] + djk[k]);
+                    }
+                    const float dq = q_ijkl + d_large;
+                    if (dq > s.cutoff) mask |= 1u << (k * TILE + l);
+                } else {
+                    float d_large = -36.8f;
+                    if (s.do_k) {
+                        d_large = fmaxf(d_large, dik[k]);
+                        d_large = fmaxf(d_large, djk[k]);
+                        d_large = fmaxf(d_large, dil[l]);
+                        d_large = fmaxf(d_large, djl[l]);
+                    }
+                    if (s.do_j) {
+                        d_large = fmaxf(d_large, d_ij);
+                        d_large = fmaxf(d_large, dkl[l]);
+                    }
+                    const float dq = q_ijkl + d_large;
+                    if (dq > s.cutoff) mask |= 1u << (k * TILE + l);
                 }
-                if (s.do_j) {
-                    d_large = fmaxf(d_large, d_ij);
-                    d_large = fmaxf(d_large, dkl[l]);
-                }
-                const float dq = q_ijkl + d_large;
-                if (dq > s.cutoff) mask |= 1u << (k * TILE + l);
             }
         }
     }
@@ -186,7 +218,7 @@ __global__ void __launch_bounds__(256) screen_tasks_kernel(const ScreenArgs s)
     const int total = __shfl_sync(0xffffffffu, incl, 31);
     if (total == 0) return;
     if (lane == 31) atomicAdd(s.qcount, (unsigned long long)total);
-    if (s.tile_mode) {
+    if (!GRAD && s.tile_mode) {
         // one 16-byte record per thread with survivors
         const unsigned has = __ballot_sync(0xffffffffu, mask != 0);
         unsigned base = 0;
@@ -209,6 +241,21 @@ __global__ void __launch_bounds__(256) screen_tasks_kernel(const ScreenArgs s)
         s.queue[pos++] = make_ushort4((unsigned short)ish, (unsigned short)jsh,
                                       (unsigned short)(tk * TILE + (b >> 2)), (unsigned short)(tl * TILE + (b & 3)));
     }
+}
+
+// ------------------------------------------------------------------ energy gradient
+// Per-shell accumulator -> (natm, 3) gradient; shell_atom[s] = -1 for pads.  One thread per
+// (atom, xyz), a fixed summation order (deterministic for a given accumulator).
+__global__ void grad_shell_to_atom_kernel(const double* __restrict__ gshell, const int* __restrict__ shell_atom, int nbas,
+                                          int natm, double* __restrict__ grad)
+{
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= 3 * natm) return;
+    const int atom = t / 3, d = t - 3 * atom;
+    double s = 0.0;
+    for (int sh = 0; sh < nbas; sh++)
+        if (shell_atom[sh] == atom) s += gshell[3 * sh + d];
+    grad[t] = s;
 }
 
 // ------------------------------------------------------------------ primitive-pair tables

@@ -223,6 +223,14 @@ class BasisLayout:
         return np.where(dec >= 0, loc[np.maximum(dec, 0)], -1).astype(np.int32)
 
     @property
+    def shell_atom(self) -> np.ndarray:
+        """(nbasis,) atom of each kernel-side shell, -1 for pads; split and decontracted shells map to
+        the atom of their parent shell."""
+        out = np.full(self.nbasis, -1, dtype=np.int32)
+        out[~self.pad_id] = np.asarray(self.splitted_mol._bas)[self.to_split_map[~self.pad_id], ATOM_OF]
+        return out
+
+    @property
     def mol_nao(self) -> int:
         return int(self._mol_dec_ao_loc()[-1])
 
