@@ -132,6 +132,21 @@ int jqc_jk_energy_grad(jqc_engine* eng, const double* dm_dev, double j_factor, d
                        double omega, double cutoff, const int* shell_atom, int natm, double* grad_dev,
                        long long* quartets, void* stream);
 
+/* Spin-unrestricted form of jqc_jk_energy_grad for two symmetric spin densities Da, Db (dm_dev:
+ * 2 x mol_nao x mol_nao, Da then Db, molecule AO basis, FP64) and Dt = Da + Db:
+ *     E_U(R) = (j_factor / 2) tr(Dt J[Dt]) - (k_factor / 2) [tr(Da K[Da]) + tr(Db K[Db])]
+ * with J, K exactly what jqc_get_jk(n_dm = 2, hermi = 1, omega) returns for [Da, Db]
+ * (J[Dt] = J[Da] + J[Db]).  With Da = Db = D / 2 this is the E_jk(D) of jqc_jk_energy_grad.  One pass
+ * over the derivative integrals serves both spins.  UHF: j_factor = k_factor = 1; UKS hybrid:
+ * k_factor = hyb; the long-range part of a range-separated hybrid is a second call with omega > 0,
+ * j_factor = 0, k_factor = alpha - hyb.  Quartets are screened with q_ij + q_kl + max(dJ_ij + dJ_kl
+ * [j_factor != 0], dS_ik + dS_jl, dS_il + dS_jk [k_factor != 0]) > log(cutoff) in float32 logs, where
+ * dJ pools |Dt| and dS pools max_s |Ds|.  grad_dev, shell_atom, natm, quartets, shards, JQC_EINVAL
+ * cases and the untouched state of the last J/K build are as for jqc_jk_energy_grad. */
+int jqc_jk_energy_grad_uhf(jqc_engine* eng, const double* dm_dev, double j_factor, double k_factor,
+                           double omega, double cutoff, const int* shell_atom, int natm, double* grad_dev,
+                           long long* quartets, void* stream);
+
 /* Accounting of the last build (synchronises the engine's device).  counts: 625 entries,
  * quartets evaluated per class key ((li*5+lj)*5+lk)*5+ll; prim_weighted: the same weighted by
  * npi*npj*npk*npl (for the algorithmic FLOP model of SURVEY 8d); launches: kernels enqueued. */

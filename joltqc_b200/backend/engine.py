@@ -171,16 +171,31 @@ class JKEngine:
         d = self._dev(dm)
         if d.ndim != 2 or d.shape[0] != self.mol_nao or d.shape[1] != self.mol_nao:
             raise ValueError(f"dm has shape {tuple(d.shape)}, expected ({self.mol_nao}, {self.mol_nao})")
+        return self._energy_grad(self.L.jqc_jk_energy_grad, d, shell_atom, natm, j_factor, k_factor, omega, cutoff,
+                                 group, count)
+
+    def jk_energy_grad_uhf(self, dm, shell_atom, natm, j_factor=1.0, k_factor=1.0, omega=None, cutoff=1e-13,
+                           group=None, count=False):
+        """Nuclear gradient of E_U = (j_factor/2) tr(Dt J[Dt]) - (k_factor/2) [tr(Da K[Da]) + tr(Db K[Db])]
+        for two symmetric spin densities ``dm = [Da, Db]`` (2 x mol_nao x mol_nao, molecule AO basis) and
+        Dt = Da + Db, in one pass over the derivative integrals (jqc_jk_energy_grad_uhf).  Sharding and
+        ``count`` as in jk_energy_grad."""
+        d = self._dev(dm)
+        if d.ndim != 3 or tuple(d.shape) != (2, self.mol_nao, self.mol_nao):
+            raise ValueError(f"dm has shape {tuple(d.shape)}, expected (2, {self.mol_nao}, {self.mol_nao})")
+        return self._energy_grad(self.L.jqc_jk_energy_grad_uhf, d, shell_atom, natm, j_factor, k_factor, omega,
+                                 cutoff, group, count)
+
+    def _energy_grad(self, fn, d, shell_atom, natm, j_factor, k_factor, omega, cutoff, group, count):
         sa = np.ascontiguousarray(shell_atom, dtype=np.int32)
         if sa.shape != (self.nbas,):
             raise ValueError(f"shell_atom has shape {sa.shape}, expected ({self.nbas},)")
         out = torch.empty((int(natm), 3), dtype=torch.float64, device=self.device)
         nq = ctypes.c_longlong(0)
         with torch.cuda.device(self.device):
-            _lib.check(self.L.jqc_jk_energy_grad(self.h, d.data_ptr(), float(j_factor), float(k_factor),
-                                                 0.0 if omega is None else float(omega), float(cutoff),
-                                                 _ptr(sa, ctypes.c_int), int(natm), out.data_ptr(),
-                                                 ctypes.byref(nq) if count else None, self._stream()))
+            _lib.check(fn(self.h, d.data_ptr(), float(j_factor), float(k_factor), 0.0 if omega is None else float(omega),
+                          float(cutoff), _ptr(sa, ctypes.c_int), int(natm), out.data_ptr(),
+                          ctypes.byref(nq) if count else None, self._stream()))
             if count:
                 self.last_grad_quartets = int(nq.value)
             if getattr(self, "_world", 1) > 1:

@@ -13,7 +13,7 @@ EXPORTS = [
     "jqc_engine_create", "jqc_engine_destroy", "jqc_last_error", "jqc_engine_set_shard", "jqc_q_matrix",
     "jqc_dm_from_mol", "jqc_dm_to_mol", "jqc_get_jk", "jqc_get_jk_host", "jqc_build_partial", "jqc_finalize",
     "jqc_last_stats", "jqc_set_profiling", "jqc_last_class_ms", "jqc_engine_nao", "jqc_engine_mol_nao",
-    "jqc_fp64_peak_probe", "jqc_last_band_stats", "jqc_jk_energy_grad",
+    "jqc_fp64_peak_probe", "jqc_last_band_stats", "jqc_jk_energy_grad", "jqc_jk_energy_grad_uhf",
 ]
 
 
@@ -62,6 +62,8 @@ def load():
     L.jqc_finalize.argtypes = [vp, dp, dp, vp]
     L.jqc_jk_energy_grad.argtypes = [vp, dp, cd, cd, cd, cd, ctypes.POINTER(ci), ci, dp,
                                      ctypes.POINTER(ctypes.c_longlong), vp]
+    L.jqc_jk_energy_grad_uhf.argtypes = [vp, dp, cd, cd, cd, cd, ctypes.POINTER(ci), ci, dp,
+                                         ctypes.POINTER(ctypes.c_longlong), vp]
     L.jqc_last_stats.argtypes = [vp, ctypes.POINTER(ctypes.c_longlong), ctypes.POINTER(ctypes.c_longlong),
                                  ctypes.POINTER(ci)]
     L.jqc_last_band_stats.argtypes = [vp, ctypes.POINTER(ctypes.c_longlong), ctypes.POINTER(ctypes.c_float)]

@@ -115,6 +115,7 @@ struct jqc_engine {
     DevBuf<unsigned long long> d_gqcounts;
     DevBuf<double> d_gshell;
     DevBuf<int> d_gatom;
+    DevBuf<float> d_glogdj;   // pooled log density of the J term (Da + Db) of the spin-unrestricted gradient
     int rank = 0, world = 1;
     // task format for blocks of <= 81 integrals: 0 flat quartets (default), 1 4x4 tile records.
     // Both were measured in round 1 (profiles/README.md); JQC_SMALL_TILES=1 selects the tile kernel.
@@ -741,14 +742,17 @@ extern "C" int jqc_build_partial(jqc_engine* e, const double* dm_dev, int n_dm, 
 }
 
 // ---------------------------------------------------------------------------------------
-// Nuclear gradient of E_jk = (j_factor/2) tr(D J[D]) - (k_factor/4) tr(D K[D]) (include/joltqc_b200.h).
+// Nuclear gradient of the J/K energy (include/joltqc_b200.h), shared by both entry points:
+//   nspin = 1: E_jk = (j_factor/2) tr(D J[D]) - (k_factor/4) tr(D K[D]) for one density D;
+//   nspin = 2: E_U = (j_factor/2) tr(Dt J[Dt]) - (k_factor/2) sum_s tr(Ds K[Ds]) for the spin densities
+//              Da, Db (dm_dev holds both) and Dt = Da + Db.
 // Same front end as a J/K build (transform in, pooling, active tile lists, chunked group-quartet loop
 // with the device queue), on the quartet-list path only.  The density scratch, the pooled density and the
 // queue are shared with the J/K builds (stream-ordered); the [J || K] buffer, the chunk records and the
 // task counters that jqc_finalize and jqc_last_stats read are not touched.
-extern "C" int jqc_jk_energy_grad(jqc_engine* e, const double* dm_dev, double j_factor, double k_factor, double omega,
-                                  double cutoff, const int* shell_atom, int natm, double* grad_dev, long long* quartets,
-                                  void* stream)
+static int jk_energy_grad(jqc_engine* e, const double* dm_dev, int nspin, double j_factor, double k_factor,
+                          double omega, double cutoff, const int* shell_atom, int natm, double* grad_dev,
+                          long long* quartets, void* stream)
 {
     if (!e || !dm_dev || !shell_atom || !grad_dev) return fail(JQC_EINVAL, "null argument");
     if (omega < 0) return fail(JQC_EINVAL, "short ranged J/K not supported");
@@ -765,27 +769,43 @@ extern "C" int jqc_jk_energy_grad(jqc_engine* e, const double* dm_dev, double j_
 
     const int nao = e->nao, nbas = e->nbas, npairs = e->npairs();
     const size_t nao2 = (size_t)nao * nao;
-    CU(e->d_dm.ensure(std::max<size_t>(nao2, 1)));
+    // kernel-side densities: D, or [Da | Db | Dt]
+    CU(e->d_dm.ensure(std::max<size_t>((nspin == 1 ? 1 : 3) * nao2, 1)));
     CU(e->d_cond.ensure((size_t)nbas * nbas));
     CU(e->d_logd.ensure((size_t)nbas * nbas));
+    if (nspin == 2) CU(e->d_glogdj.ensure((size_t)nbas * nbas));
     CU(e->d_gcounters.ensure(MAX_CHUNKS));
     CU(e->d_gqcounts.ensure(MAX_CHUNKS));
     CU(e->d_gshell.ensure((size_t)nbas * 3));
     CU(e->d_gatom.ensure(nbas));
     CU(cudaMemcpyAsync(e->d_gatom.p, shell_atom, nbas * sizeof(int), cudaMemcpyHostToDevice, st));
 
-    // 1. AO transform in, 2. pooling (hermi = 1), log, global max, 3. active tile counts (quadratic in D)
-    rc = launch_from_mol(e, dm_dev, 1, e->d_dm.p, false, st);
+    // 1. AO transform in (and Dt = Da + Db), 2. pooling (hermi = 1), log, global max: d pools max_s |Ds|
+    // (the K terms), dJ pools Dt (the J term); both logs raise the one global maximum.  3. active tile
+    // counts (quadratic in D).
+    rc = launch_from_mol(e, dm_dev, nspin, e->d_dm.p, false, st);
     if (rc) return rc;
-    dm_pool_kernel<<<nbas, 256, nbas * sizeof(float), st>>>(e->d_dm.p, 1, nao, nbas, e->d_ao_loc.p, e->d_ao2shell.p,
-                                                          e->d_cond.p);
-    CU(cudaGetLastError());
+    if (nspin == 2) {
+        const unsigned blocks = (unsigned)std::min<size_t>((nao2 + 255) / 256, 65535u * 16);
+        dm_spin_sum_kernel<<<blocks, 256, 0, st>>>(e->d_dm.p, e->d_dm.p + nao2, e->d_dm.p + 2 * nao2, nao2);
+        CU(cudaGetLastError());
+    }
     {
         const int neg_inf_ordered = (int)0xFF800000 ^ 0x7FFFFFFF;   // float_to_ordered(-inf)
         CU(cudaMemcpyAsync(e->d_logmax.p, &neg_inf_ordered, sizeof(int), cudaMemcpyHostToDevice, st));
         dim3 grid(nbas, (nbas + 127) / 128);
+        dm_pool_kernel<<<nbas, 256, nbas * sizeof(float), st>>>(e->d_dm.p, nspin, nao, nbas, e->d_ao_loc.p,
+                                                              e->d_ao2shell.p, e->d_cond.p);
+        CU(cudaGetLastError());
         dm_log_kernel<<<grid, 128, 0, st>>>(e->d_cond.p, nbas, 1, e->d_logd.p, e->d_logmax.p);
         CU(cudaGetLastError());
+        if (nspin == 2) {
+            dm_pool_kernel<<<nbas, 256, nbas * sizeof(float), st>>>(e->d_dm.p + 2 * nao2, 1, nao, nbas, e->d_ao_loc.p,
+                                                                  e->d_ao2shell.p, e->d_cond.p);
+            CU(cudaGetLastError());
+            dm_log_kernel<<<grid, 128, 0, st>>>(e->d_cond.p, nbas, 1, e->d_glogdj.p, e->d_logmax.p);
+            CU(cudaGetLastError());
+        }
     }
     active_tiles_grad_kernel<<<(npairs + 127) / 128, 128, 0, st>>>(qd->tiles_q.p, qd->list_off.p, npairs, e->d_logmax.p,
                                                                   e->d_nact.p);
@@ -827,6 +847,7 @@ extern "C" int jqc_jk_energy_grad(jqc_engine* e, const double* dm_dev, double j_
             s.nbas = nbas;
             s.q = qd->q.p;
             s.logd = e->d_logd.p;
+            s.logd_j = nspin == 1 ? e->d_logd.p : e->d_glogdj.p;
             s.log_max_ordered = e->d_logmax.p;
             s.tiles_ij = qd->tiles.p + qd->h_list_off[pij];
             s.tiles_kl = qd->tiles.p + qd->h_list_off[pkl];
@@ -854,13 +875,15 @@ extern "C" int jqc_jk_energy_grad(jqc_engine* e, const double* dm_dev, double j_
             a.npi = e->gnp[gi]; a.npj = e->gnp[gj]; a.npk = e->gnp[gk]; a.npl = e->gnp[gl];
             a.basis = e->d_basis.p;
             a.dm = e->d_dm.p;
+            a.dm_b = nspin == 1 ? nullptr : e->d_dm.p + nao2;
+            a.dm_t = nspin == 1 ? nullptr : e->d_dm.p + 2 * nao2;
             a.j_factor4 = 4.0 * j_factor;
-            a.k_factor = k_factor;
+            a.k_factor = nspin == 1 ? k_factor : 2.0 * k_factor;
             a.omega = omega;
             a.quartets = e->d_queue.p;
             a.ntasks = e->d_gcounters.p + cid;
             a.gshell = e->d_gshell.p;
-            CU(jk_grad_launch(li, lj, lk, ll, a, e->nsm, st));
+            CU(jk_grad_launch(li, lj, lk, ll, nspin, a, e->nsm, st));
         }
     }
     // 5. shells -> atoms
@@ -875,6 +898,20 @@ extern "C" int jqc_jk_energy_grad(jqc_engine* e, const double* dm_dev, double j_
         *quartets = n;
     }
     return JQC_OK;
+}
+
+extern "C" int jqc_jk_energy_grad(jqc_engine* e, const double* dm_dev, double j_factor, double k_factor, double omega,
+                                  double cutoff, const int* shell_atom, int natm, double* grad_dev, long long* quartets,
+                                  void* stream)
+{
+    return jk_energy_grad(e, dm_dev, 1, j_factor, k_factor, omega, cutoff, shell_atom, natm, grad_dev, quartets, stream);
+}
+
+extern "C" int jqc_jk_energy_grad_uhf(jqc_engine* e, const double* dm_dev, double j_factor, double k_factor,
+                                      double omega, double cutoff, const int* shell_atom, int natm, double* grad_dev,
+                                      long long* quartets, void* stream)
+{
+    return jk_energy_grad(e, dm_dev, 2, j_factor, k_factor, omega, cutoff, shell_atom, natm, grad_dev, quartets, stream);
 }
 
 extern "C" int jqc_finalize(jqc_engine* e, double* vj_dev, double* vk_dev, void* stream)

@@ -109,6 +109,7 @@ struct ScreenArgs {
     int nbas;
     const float* __restrict__ q;
     const float* __restrict__ logd;
+    const float* __restrict__ logd_j;    // GRAD only: pooled log density of the J term (logd for one density)
     const int* __restrict__ log_max_ordered;
     const int* __restrict__ tiles_ij;    // tile ids ti*nt+tj, q-descending
     const int* __restrict__ tiles_kl;
@@ -131,8 +132,10 @@ struct ScreenArgs {
 // (jqc/backend/jk/screen_jk_tasks.cu:196-261), compacted per warp with one atomic.
 // A warp holds 32 kl tiles for a single (i,j), so its output run shares i and j.
 // GRAD selects the screen of the J/K energy gradient, whose weights are products of two density
-// blocks: q_ij + q_kl + max(d_ij + d_kl [J], d_ik + d_jl, d_il + d_jk [K]) > cutoff, with the tile
-// prefilter on 2 log max|D| (flat quartet records only).
+// blocks: q_ij + q_kl + max(dJ_ij + dJ_kl [J], d_ik + d_jl, d_il + d_jk [K]) > cutoff, with the tile
+// prefilter on 2 log max|D| (flat quartet records only).  dJ (logd_j) is the pooled density of the J
+// term: logd itself for one density, the pooled Da + Db for two spin densities, where logd pools
+// max_s |Ds| and log max|D| is the larger of the two maxima.
 template <bool GRAD>
 __global__ void __launch_bounds__(256) screen_tasks_kernel(const ScreenArgs s)
 {
@@ -168,13 +171,14 @@ __global__ void __launch_bounds__(256) screen_tasks_kernel(const ScreenArgs s)
         const float4 d_jl = *reinterpret_cast<const float4*>(s.logd + (size_t)jsh * nbas + lsh0);
         const float dik[4] = {d_ik.x, d_ik.y, d_ik.z, d_ik.w}, djk[4] = {d_jk.x, d_jk.y, d_jk.z, d_jk.w};
         const float dil[4] = {d_il.x, d_il.y, d_il.z, d_il.w}, djl[4] = {d_jl.x, d_jl.y, d_jl.z, d_jl.w};
-        const float d_ij = s.logd[(size_t)ish * nbas + jsh];
+        const float* __restrict__ logd_j = GRAD ? s.logd_j : s.logd;
+        const float d_ij = logd_j[(size_t)ish * nbas + jsh];
         const long long bas_ij = (long long)ish * nbas + jsh;
 #pragma unroll
         for (int k = 0; k < TILE; k++) {
             const int ksh = ksh0 + k;
             const float4 qk = *reinterpret_cast<const float4*>(s.q + (size_t)ksh * nbas + lsh0);
-            const float4 dk = *reinterpret_cast<const float4*>(s.logd + (size_t)ksh * nbas + lsh0);
+            const float4 dk = *reinterpret_cast<const float4*>(logd_j + (size_t)ksh * nbas + lsh0);
             const float qkl[4] = {qk.x, qk.y, qk.z, qk.w}, dkl[4] = {dk.x, dk.y, dk.z, dk.w};
 #pragma unroll
             for (int l = 0; l < TILE; l++) {
@@ -244,6 +248,14 @@ __global__ void __launch_bounds__(256) screen_tasks_kernel(const ScreenArgs s)
 }
 
 // ------------------------------------------------------------------ energy gradient
+// Dt = Da + Db of the spin-unrestricted gradient (kernel-side densities, n = nao^2 elements each)
+__global__ void dm_spin_sum_kernel(const double* __restrict__ da, const double* __restrict__ db, double* __restrict__ dt,
+                                   size_t n)
+{
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
+        dt[i] = da[i] + db[i];
+}
+
 // Per-shell accumulator -> (natm, 3) gradient; shell_atom[s] = -1 for pads.  One thread per
 // (atom, xyz), a fixed summation order (deterministic for a given accumulator).
 __global__ void grad_shell_to_atom_kernel(const double* __restrict__ gshell, const int* __restrict__ shell_atom, int nbas,

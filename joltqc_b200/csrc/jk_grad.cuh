@@ -15,6 +15,12 @@
 // streams: per primitive quartet and root only nine partial sums (three centres x xyz) are kept; the
 // 2a factors are applied per primitive quartet, the lowered terms (no exponent) once per quartet.
 // Each quartet adds its four centres' 3-vectors into a per-shell nbas x 3 accumulator.
+//
+// NSPIN = 2 is the spin-unrestricted energy for two symmetric spin densities Da, Db (Dt = Da + Db)
+//     E_U = (j_factor / 2) tr(Dt J[Dt]) - (k_factor / 2) [tr(Da K[Da]) + tr(Db K[Db])]
+// with the weight
+//     W_n = 4 j_factor Dt_ij Dt_kl - 2 k_factor sum_s (Ds_ik Ds_jl + Ds_il Ds_jk);
+// everything downstream of the weight is the same as for NSPIN = 1.
 #pragma once
 #include "jk_1q1t.cuh"
 
@@ -24,22 +30,34 @@ struct GradArgs {
     int nao;
     int npi, npj, npk, npl;
     const double* __restrict__ basis;     // nbas x 12 packed shell records
-    const double* __restrict__ dm;        // nao x nao kernel-side cartesian density (symmetric)
+    const double* __restrict__ dm;        // nao x nao kernel-side cartesian density (symmetric); NSPIN = 2: Da
     double j_factor4;                     // 4 * j_factor
-    double k_factor;
+    double k_factor;                      // k_factor; NSPIN = 2: 2 * k_factor
     double omega;                         // 0: Coulomb, > 0: long-range erf
     const ushort4* __restrict__ quartets;
     const unsigned* __restrict__ ntasks;  // device counter written by the task generator
     double* __restrict__ gshell;          // nbas x 3, accumulated
+    const double* __restrict__ dm_b;      // NSPIN = 2: Db (nao x nao, symmetric)
+    const double* __restrict__ dm_t;      // NSPIN = 2: Dt = Da + Db
 };
 
 // W_n of one cartesian component (absolute AO indices)
+template <int NSPIN>
 __device__ __forceinline__ double grad_weight(const GradArgs& a, int i, int j, int k, int l)
 {
-    const double* __restrict__ dm = a.dm;
     const size_t n = (size_t)a.nao;
-    return fma(a.j_factor4 * __ldg(dm + i * n + j), __ldg(dm + k * n + l),
-               -a.k_factor * fma(__ldg(dm + i * n + k), __ldg(dm + j * n + l), __ldg(dm + i * n + l) * __ldg(dm + j * n + k)));
+    if constexpr (NSPIN == 1) {
+        const double* __restrict__ dm = a.dm;
+        return fma(a.j_factor4 * __ldg(dm + i * n + j), __ldg(dm + k * n + l),
+                   -a.k_factor * fma(__ldg(dm + i * n + k), __ldg(dm + j * n + l), __ldg(dm + i * n + l) * __ldg(dm + j * n + k)));
+    } else {
+        const double* __restrict__ da = a.dm;
+        const double* __restrict__ db = a.dm_b;
+        const double* __restrict__ dt = a.dm_t;
+        const double ka = fma(__ldg(da + i * n + k), __ldg(da + j * n + l), __ldg(da + i * n + l) * __ldg(da + j * n + k));
+        const double kb = fma(__ldg(db + i * n + k), __ldg(db + j * n + l), __ldg(db + i * n + l) * __ldg(db + j * n + k));
+        return fma(a.j_factor4 * __ldg(dt + i * n + j), __ldg(dt + k * n + l), -a.k_factor * (ka + kb));
+    }
 }
 
 template <int LI, int LJ, int LK, int LL>
@@ -53,7 +71,7 @@ struct GradShape {
     static constexpr bool SMALL = 3 * G::GSIZE + S::N <= 128;
 };
 
-template <int LI, int LJ, int LK, int LL, bool SMALL, int NT>
+template <int LI, int LJ, int LK, int LL, bool SMALL, int NT, int NSPIN>
 __global__ void __launch_bounds__(NT) jk_grad_kernel(const GradArgs a)
 {
     using S = QuartetShape<LI, LJ, LK, LL>;
@@ -94,7 +112,7 @@ __global__ void __launch_bounds__(NT) jk_grad_kernel(const GradArgs a)
 #pragma unroll
             for (int k = 0; k < NFK; k++)
 #pragma unroll
-            for (int l = 0; l < NFL; l++) w[((i * NFJ + j) * NFK + k) * NFL + l] = grad_weight(a, i0 + i, j0 + j, k0 + k, l0 + l);
+            for (int l = 0; l < NFL; l++) w[((i * NFJ + j) * NFK + k) * NFL + l] = grad_weight<NSPIN>(a, i0 + i, j0 + j, k0 + k, l0 + l);
         }
 
         const double rjri[3] = {rj.x - ri.x, rj.y - ri.y, rj.z - ri.z};
@@ -180,7 +198,7 @@ __global__ void __launch_bounds__(NT) jk_grad_kernel(const GradArgs a)
                         const double* __restrict__ gz = g + 2 * GS;
                         double wn;
                         if constexpr (SMALL) wn = w[((i * NFJ + j) * NFK + k) * NFL + l];
-                        else wn = grad_weight(a, i0 + i, j0 + j, k0 + k, l0 + l);
+                        else wn = grad_weight<NSPIN>(a, i0 + i, j0 + j, k0 + k, l0 + l);
                         const double x = gx[ax], y = gyv[ay], z = gz[az];
                         const double wyz = wn * y * z, wxz = wn * x * z, wxy = wn * x * y;
                         e = fma(wyz, x, e);
@@ -224,8 +242,9 @@ __global__ void __launch_bounds__(NT) jk_grad_kernel(const GradArgs a)
 }
 
 // Launchers, one translation unit per bra class (jk_grad_inst.cu).  Same class order as jk_launch:
-// li >= lj, li >= lk, lk >= ll.
-#define JQC_GRAD_DECL(I, J) cudaError_t jk_grad_launch_##I##_##J(int lk, int ll, const GradArgs& a, int nsm, cudaStream_t st);
+// li >= lj, li >= lk, lk >= ll.  nspin: 1 (one density) or 2 (spin-unrestricted).
+#define JQC_GRAD_DECL(I, J) \
+    cudaError_t jk_grad_launch_##I##_##J(int lk, int ll, int nspin, const GradArgs& a, int nsm, cudaStream_t st);
 JQC_GRAD_DECL(0, 0)
 JQC_GRAD_DECL(1, 0) JQC_GRAD_DECL(1, 1)
 JQC_GRAD_DECL(2, 0) JQC_GRAD_DECL(2, 1) JQC_GRAD_DECL(2, 2)
@@ -233,9 +252,9 @@ JQC_GRAD_DECL(3, 0) JQC_GRAD_DECL(3, 1) JQC_GRAD_DECL(3, 2) JQC_GRAD_DECL(3, 3)
 JQC_GRAD_DECL(4, 0) JQC_GRAD_DECL(4, 1) JQC_GRAD_DECL(4, 2) JQC_GRAD_DECL(4, 3) JQC_GRAD_DECL(4, 4)
 #undef JQC_GRAD_DECL
 
-inline cudaError_t jk_grad_launch(int li, int lj, int lk, int ll, const GradArgs& a, int nsm, cudaStream_t st)
+inline cudaError_t jk_grad_launch(int li, int lj, int lk, int ll, int nspin, const GradArgs& a, int nsm, cudaStream_t st)
 {
-#define JQC_CALL(I, J) if (li == I && lj == J) return jk_grad_launch_##I##_##J(lk, ll, a, nsm, st);
+#define JQC_CALL(I, J) if (li == I && lj == J) return jk_grad_launch_##I##_##J(lk, ll, nspin, a, nsm, st);
     JQC_CALL(0, 0)
     JQC_CALL(1, 0) JQC_CALL(1, 1)
     JQC_CALL(2, 0) JQC_CALL(2, 1) JQC_CALL(2, 2)

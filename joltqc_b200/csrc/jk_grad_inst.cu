@@ -1,6 +1,6 @@
 // One translation unit per bra class (JQC_LI >= JQC_LJ), compiled with -DJQC_LI=.. -DJQC_LJ=..
-// Instantiates the J/K energy-gradient kernel (jk_grad.cuh) for every ket class lk <= li, ll <= lk
-// and exports one launcher.
+// Instantiates the J/K energy-gradient kernel (jk_grad.cuh) for every ket class lk <= li, ll <= lk,
+// one density (NSPIN = 1) and two spin densities (NSPIN = 2), and exports one launcher.
 #include <atomic>
 
 #include "jk_grad.cuh"
@@ -10,12 +10,12 @@ namespace jqc {
 // occupancy per device ordinal, computed on first use (as in jk_inst.cu)
 constexpr int JQC_GRAD_MAX_DEVICES = 64;
 
-template <int LK, int LL>
+template <int LK, int LL, int NSPIN>
 static cudaError_t grad_launch_one(const GradArgs& a, int nsm, cudaStream_t st)
 {
     constexpr bool SMALL = GradShape<JQC_LI, JQC_LJ, LK, LL>::SMALL;
     constexpr int NT = 128;
-    auto kern = jk_grad_kernel<JQC_LI, JQC_LJ, LK, LL, SMALL, NT>;
+    auto kern = jk_grad_kernel<JQC_LI, JQC_LJ, LK, LL, SMALL, NT, NSPIN>;
     static std::atomic<int> cache[JQC_GRAD_MAX_DEVICES];
     int dev = 0;
     cudaError_t e = cudaGetDevice(&dev);
@@ -37,11 +37,12 @@ static cudaError_t grad_launch_one(const GradArgs& a, int nsm, cudaStream_t st)
 
 // (templated on a dummy so that the discarded `if constexpr` branches are not instantiated)
 template <int Z>
-static cudaError_t grad_dispatch(int lk, int ll, const GradArgs& a, int nsm, cudaStream_t st)
+static cudaError_t grad_dispatch(int lk, int ll, int nspin, const GradArgs& a, int nsm, cudaStream_t st)
 {
-#define CASE(K, L)                                                       \
-    if constexpr (K + Z <= JQC_LI && L <= K) {                           \
-        if (lk == K && ll == L) return grad_launch_one<K, L>(a, nsm, st); \
+#define CASE(K, L)                                                                  \
+    if constexpr (K + Z <= JQC_LI && L <= K) {                                      \
+        if (lk == K && ll == L)                                                     \
+            return nspin == 1 ? grad_launch_one<K, L, 1>(a, nsm, st) : grad_launch_one<K, L, 2>(a, nsm, st); \
     }
     CASE(0, 0)
     CASE(1, 0) CASE(1, 1)
@@ -52,9 +53,10 @@ static cudaError_t grad_dispatch(int lk, int ll, const GradArgs& a, int nsm, cud
     return cudaErrorInvalidValue;
 }
 
-cudaError_t JQC_CAT(jk_grad_launch_, JQC_LI, JQC_LJ)(int lk, int ll, const GradArgs& a, int nsm, cudaStream_t st)
+cudaError_t JQC_CAT(jk_grad_launch_, JQC_LI, JQC_LJ)(int lk, int ll, int nspin, const GradArgs& a, int nsm, cudaStream_t st)
 {
-    return grad_dispatch<0>(lk, ll, a, nsm, st);
+    if (nspin != 1 && nspin != 2) return cudaErrorInvalidValue;
+    return grad_dispatch<0>(lk, ll, nspin, a, nsm, st);
 }
 
 }  // namespace jqc
